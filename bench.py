@@ -2,6 +2,7 @@
 """Benchmark of the WeKws streaming KWS forward path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--no-extras]
+                    [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1]): the `mdtc` model (hidden 64, 1+4x4 DS-dilated blocks, k=5),
 80-dim features, B = 1024 concurrent streams per GPU, chunk T = 40 frames, streaming caches (B,64,244)
@@ -31,6 +32,10 @@ frames.  Metric: audio-hours/sec = frames/sec / 360000 (100 frames per second).
 Multi-GPU: streams are independent -> each rank owns its own B streams ("weak" scaling), no collective
 on the data path; torch.distributed (NCCL) is used only for the barrier and the max-over-ranks time.
 Between timed steps the working set rotates over NSETS independent stream sets (> 126 MB L2).
+--dump-outputs DIR: what the last timed step of the headline workload returned to its caller, written after the timed
+               loop as DIR/posteriors.npy (B, T, odim) and DIR/cache.npy (the streaming cache), float32, rank 0.  At
+               most DUMP_BYTES in all: an array that does not fit keeps a fixed, seeded sample of its streams.  Inputs
+               and weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -60,6 +65,7 @@ WORKLOADS = {
 EXTRAS = ["gru_b512_t1", "tcn_b1024_t40", "ds_tcn_b1024_t40", "pcm_e2e_1250x1s"]
 PCM_SAMPLES = 16000
 NSETS = 4
+DUMP_BYTES = 64 * 10 ** 6
 METRIC = "audio-hours/sec KWS scoring (frames/sec / 360000)"
 DTYPE = "f32 I/O, bf16x3 tensor GEMMs (fp32 accumulate, ~2^-17; GRU and front-end: fp32 FMA)"
 
@@ -278,6 +284,25 @@ def workload_config(workload, gpus):
 
 
 # ------------------------------------------------------------------------------------------- our arm
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> (tensor, index of its stream dimension), written in this order as out_dir/<name>.npy (float32).
+    An array larger than what is left of DUMP_BYTES keeps the streams torch.randperm(n, generator seeded with 0)[:k],
+    in ascending order, for the largest k that fits."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES
+    for name, (t, dim) in arrays.items():
+        a = t.detach().float().cpu()
+        n = a.shape[dim]
+        k = min(n, left // (4 * a.numel() // n))
+        if k < n:
+            keep = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:k].sort().values
+            a = a.index_select(dim, keep)
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+        left -= 4 * a.numel()
+
+
 class Runner:
     def __init__(self, dev, rank, world, dist):
         self.dev, self.rank, self.world, self.dist = dev, rank, world, dist
@@ -296,9 +321,10 @@ class Runner:
             self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX if op == "max" else self.dist.ReduceOp.SUM)
         return float(t.item())
 
-    def run(self, workload, steps, warmup, min_region_s=0.0):
+    def run(self, workload, steps, warmup, min_region_s=0.0, dump_dir=None):
         """value / latency / e2e / roofline of one workload.  steps, warmup: the device-resident timed loop (exactly
-        as given when min_region_s == 0; extras pass min_region_s to size the loop by time instead)."""
+        as given when min_region_s == 0; extras pass min_region_s to size the loop by time instead).  dump_dir: where
+        dump_outputs() writes what the last timed step returned."""
         import torch
         from wekws_b200 import _native, init_model, model_config, synth
         dev, rank, world = self.dev, self.rank, self.world
@@ -321,12 +347,15 @@ class Runner:
             feats = [synth.features(B, T, idim, seed=4321 + rank * 17 + s).to(dev) for s in range(NSETS)]
             caches = [torch.zeros(cshape, device=dev) for _ in range(NSETS)]
 
+        last = [None]          # (posteriors, cache) the latest step returned
+
         def step(i):
             s = i % NSETS
             if pcm_mode:
-                pipe(pcm[s])
+                last[0] = pipe(pcm[s])
             else:
-                _, caches[s] = model(feats[s], caches[s])
+                y, caches[s] = model(feats[s], caches[s])
+                last[0] = (y, caches[s])
 
         # ---------------- device-resident throughput (`value`) ------------------------------------------------
         for i in range(max(warmup, 3)):
@@ -349,6 +378,8 @@ class Runner:
         t_end.record()
         self.barrier()
         launches = _native.launch_count() - n0
+        if dump_dir is not None and rank == 0:
+            dump_outputs(dump_dir, {"posteriors": (last[0][0], 0), "cache": (last[0][1], 1 if gru else 0)})
         total_ms = self.reduce(t_begin.elapsed_time(t_end))
         fps = B * T * steps * world / (total_ms * 1e-3)
         # per-launch durations (roofline, p50/p99) from a separate pass: bracketing every step with events costs
@@ -566,7 +597,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra_workloads (BASELINE configs[2..4])")
     ap.add_argument("--cpu-budget", type=float, default=60.0, help="seconds of timed CPU work for --impl reference")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -590,7 +627,7 @@ def main():
         dist = dist_mod
         dist.init_process_group("nccl", device_id=dev)
     runner = Runner(dev, rank, world, dist)
-    main_res = runner.run(args.workload, args.steps, args.warmup)
+    main_res = runner.run(args.workload, args.steps, args.warmup, dump_dir=args.dump_outputs)
     extras = []
     if not args.no_extras and args.workload == "mdtc_b1024_t40":
         for w in EXTRAS:

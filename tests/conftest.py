@@ -10,7 +10,6 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
 
 
 def pytest_configure(config):
@@ -28,17 +27,6 @@ def pytest_collection_modifyitems(config, items):
 
 def golden(name):
     return np.load(os.path.join(GOLDEN, name + ".npz"))
-
-
-def have_reference():
-    return os.path.isdir(os.path.join(REFERENCE, "wekws"))
-
-
-def reference_init_model():
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-    from wekws.model.kws_model import init_model
-    return init_model
 
 
 @pytest.fixture(scope="session")

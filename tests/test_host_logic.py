@@ -12,7 +12,7 @@ import torch
 from oracle import kws_oracle as O
 from tests import packed_eval as PE
 from tests.cases import CASE_NAMES, build_model
-from tests.conftest import ROOT, golden, have_reference, reference_init_model
+from tests.conftest import ROOT, golden
 from wekws_b200 import Fbank, init_model, model_config, synth
 from wekws_b200 import frontend
 
@@ -249,22 +249,28 @@ def test_state_dict_schema_and_init_match_reference_golden():
     assert init_model(model_config("ds_tcn")).backbone.padding == 105
 
 
-@pytest.mark.skipif(not have_reference(), reason="/root/reference not present (GPU box)")
 @pytest.mark.parametrize("name", ["mdtc", "mdtc_small", "ds_tcn", "tcn", "gru"])
 def test_checkpoints_interchange_with_live_reference(name, tmp_path):
-    ref_init = reference_init_model()
-    import contextlib, io
-    with contextlib.redirect_stdout(io.StringIO()):
-        ref = ref_init(model_config(name))
+    """A checkpoint with exactly the reference's state_dict schema (key, shape, dtype of every entry its init_model
+    builds for the same config: tests/golden/checkpoint_schema.npz) loads strictly, and ours has that schema."""
+    g = golden("checkpoint_schema")
+    dims = iter(g[name + "_dims"].tolist())
+    schema = {k: (tuple(next(dims) for _ in range(nd)), dt)
+              for k, nd, dt in zip(g[name + "_keys"].tolist(), g[name + "_ndim"].tolist(), g[name + "_dtypes"].tolist())}
+    gen = torch.Generator().manual_seed(5)
+    ref_sd = {k: (torch.full(shape, 100, dtype=getattr(torch, dt)) if dt == "int64"
+                  else torch.randn(shape, generator=gen).to(getattr(torch, dt)))
+              for k, (shape, dt) in schema.items()}
     ours = init_model(model_config(name))
-    synth.randomize_(ref, seed=5)
     path = str(tmp_path / "ckpt.pt")
-    torch.save(ref.state_dict(), path)                      # utils/checkpoint.py:46-50
+    torch.save(ref_sd, path)                                # utils/checkpoint.py:46-50
     missing = ours.load_state_dict(torch.load(path), strict=True)   # utils/checkpoint.py:30
     assert not missing.missing_keys and not missing.unexpected_keys
-    ref.load_state_dict(ours.state_dict(), strict=True)
+    assert all(torch.equal(v, ref_sd[k]) for k, v in ours.state_dict().items())
+    # what the reference's own strict load of our state_dict checks (keys, shapes), and the dtypes
+    assert {k: (tuple(v.shape), str(v.dtype).replace("torch.", "")) for k, v in ours.state_dict().items()} == schema
     # average_model.py:77-83 turns num_batches_tracked into float: loading must still work
-    avg = {k: (v.float() if v.dtype == torch.int64 else v) for k, v in ref.state_dict().items()}
+    avg = {k: (v.float() if v.dtype == torch.int64 else v) for k, v in ref_sd.items()}
     ours.load_state_dict(avg, strict=True)
 
 
@@ -308,14 +314,14 @@ def test_cmvn_loaders(tmp_path):
     assert out.shape == (2, 6) and np.allclose(out[0, :2], [1.5, 2.5]) and np.allclose(out[1, :2], [0.5, 0.25])
 
 
-def test_patch_reference_rebinds_the_reference_factory():
+def test_patch_reference_rebinds_the_reference_factory(tmp_path):
     """patch_reference() (wekws_b200/overlay.py): with the reference importable, `wekws.model.kws_model.init_model`
     and `.KWSModel` -- the names wekws/bin/score.py:30 and average_model / stream_kws_ctc import -- become this
-    implementation; without it a stub package of the same dotted name is registered.  Run in subprocesses so the
-    live-reference tests of this session keep the unpatched module."""
+    implementation; without it a stub package of the same dotted name is registered.  The importable reference is
+    stood in for by a package of the same dotted names written to tmp_path.  Run in subprocesses so the rest of this
+    session keeps the unpatched modules."""
     import subprocess
     import sys
-    from tests.conftest import ROOT, have_reference
     code_stub = ("import sys; sys.path.insert(0, %r)\n"
                  "from wekws_b200 import patch_reference; import wekws_b200.kws_model as ours\n"
                  "assert patch_reference() is False\n"
@@ -323,14 +329,20 @@ def test_patch_reference_rebinds_the_reference_factory():
                  "assert init_model is ours.init_model and KWSModel is ours.KWSModel\n" % ROOT)
     r = subprocess.run([sys.executable, "-c", code_stub], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stderr
-    if not have_reference():
-        return
-    code_real = ("import sys; sys.path.insert(0, %r); sys.path.insert(0, '/root/reference')\n"
+    model_dir = tmp_path / "wekws" / "model"
+    model_dir.mkdir(parents=True)
+    (tmp_path / "wekws" / "__init__.py").write_text("")
+    (model_dir / "__init__.py").write_text("")
+    (model_dir / "kws_model.py").write_text("class KWSModel:\n    pass\n\n\ndef init_model(configs):\n"
+                                            "    return KWSModel()\n")
+    (model_dir / "mdtc.py").write_text("")
+    code_real = ("import sys; sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
                  "import wekws.model.kws_model as ref; orig = ref.init_model\n"
                  "from wekws_b200 import patch_reference; import wekws_b200.kws_model as ours\n"
                  "assert patch_reference() is True\n"
                  "from wekws.model.kws_model import init_model, KWSModel\n"
                  "assert init_model is ours.init_model and init_model is not orig and KWSModel is ours.KWSModel\n"
-                 "import wekws.model.mdtc  # the rest of the reference package stays importable\n" % ROOT)
+                 "import wekws.model.mdtc  # the rest of the reference package stays importable\n"
+                 % (ROOT, str(tmp_path)))
     r = subprocess.run([sys.executable, "-c", code_real], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stderr

@@ -1,12 +1,12 @@
 """Pins the CPU oracle (oracle/kws_oracle.py) to the reference: golden vectors produced by the
-real reference (oracle/make_golden.py) and, when /root/reference is present, the live code."""
+real reference (oracle/make_golden.py, oracle/make_reference_golden.py)."""
 import numpy as np
 import pytest
 import torch
 
 from oracle import kws_oracle as O
 from tests.cases import CASE_NAMES, CHUNKS, build_model
-from tests.conftest import golden, have_reference, reference_init_model
+from tests.conftest import golden
 from wekws_b200 import init_model, synth
 
 TOL_MODEL = 2e-6      # oracle uses the same ATen ops as the reference: agreement is ~1 ulp
@@ -105,40 +105,48 @@ def test_oracle_cmvn_loader_matches_golden(tmp_path):
     assert np.allclose(istd.numpy(), ref[1].astype(np.float32), rtol=0, atol=0)
 
 
-@pytest.mark.skipif(not have_reference(), reason="/root/reference not present (GPU box)")
 @pytest.mark.parametrize("case", CASE_NAMES)
 def test_oracle_matches_live_reference(case):
-    ref_init = reference_init_model()
-    cfg, ref, B = build_model(case, ref_init)
-    sd = ref.state_dict()
+    """The same input streamed three times in 23-frame chunks, cache carried, against what the reference's own
+    KWSModel returned (tests/golden/stream23.npz: every output, the cache at a fixed sample of its live entries)."""
+    g = golden("stream23")
+    cfg, sd, model, B = _oracle_model(case)
+    assert abs(synth.state_digest(model) - float(g[case + "_digest"])) < 1e-6 * float(g[case + "_digest"])
     gru = cfg["backbone"]["type"] == "gru"
-    x = synth.features(B, 23, cfg["input_dim"], seed=5, cmvn_like=ref.global_cmvn is not None)
-    c_ref = torch.zeros(cfg["backbone"]["num_layers"], B, cfg["hidden_dim"]) if gru else torch.zeros(0, 0, 0)
-    c_or = c_ref if gru else None
-    with torch.no_grad():
-        for _ in range(3):
-            y_ref, c_ref = ref(x, c_ref)
-            y_or, c_or = O.kws_forward(sd, cfg, x, c_or)
-            assert (y_ref - y_or).abs().max() <= TOL_MODEL * max(1.0, float(y_ref.abs().max()))
-            assert (c_ref - c_or).abs().max() <= 1e-5
+    x = synth.features(B, 23, cfg["input_dim"], seed=5, cmvn_like=model.global_cmvn is not None)
+    assert abs(float(x.double().sum()) - float(g[case + "_x_sum"])) <= 1e-9 * float(x.double().abs().sum())
+    c_or = torch.zeros(cfg["backbone"]["num_layers"], B, cfg["hidden_dim"]) if gru else None
+    idx = torch.from_numpy(g[case + "_cidx"])
+    for i in range(3):
+        y_ref, c_ref = torch.from_numpy(g[f"{case}_y{i}"]), torch.from_numpy(g[f"{case}_c{i}"])
+        y_or, c_or = O.kws_forward(sd, cfg, x, c_or)
+        assert y_or.shape == y_ref.shape and tuple(c_or.shape) == tuple(g[case + "_cshape"])
+        assert (y_ref - y_or).abs().max() <= TOL_MODEL * max(1.0, float(y_ref.abs().max()))
+        assert (c_ref - c_or.reshape(-1)[idx]).abs().max() <= 1e-5
 
 
-@pytest.mark.skipif(not have_reference(), reason="/root/reference not present (GPU box)")
+def _sampled_frames(g, name):
+    return tuple(g[name + "_shape"]), torch.from_numpy(g[name + "_frames"]), torch.from_numpy(g[name])
+
+
 def test_oracle_mfcc_matches_live_torchaudio():
-    import torchaudio.compliance.kaldi as kaldi
+    """Against torchaudio.compliance.kaldi.mfcc on the same audio (tests/golden/kaldi_live.npz, a fixed sample of
+    40 frames)."""
     pcm = synth.pcm_int16(1, 16000 * 2, seed=78)[0].float()
-    ref = kaldi.mfcc(pcm.unsqueeze(0), num_ceps=80, num_mel_bins=80, frame_length=25, frame_shift=10, dither=0.0,
-                     energy_floor=0.0, sample_frequency=16000)
-    assert (O.mfcc(pcm) - ref).abs().max() <= 2e-4
+    shape, frames, ref = _sampled_frames(golden("kaldi_live"), "mfcc80_seed78")
+    out = O.mfcc(pcm)
+    assert tuple(out.shape) == shape
+    assert (out[frames] - ref).abs().max() <= 2e-4
 
 
-@pytest.mark.skipif(not have_reference(), reason="/root/reference not present (GPU box)")
 def test_oracle_fbank_matches_live_torchaudio():
-    import torchaudio.compliance.kaldi as kaldi
+    """Against torchaudio.compliance.kaldi.fbank on the same audio (tests/golden/kaldi_live.npz, a fixed sample of
+    40 frames)."""
     pcm = synth.pcm_int16(1, 16000 * 3, seed=77)[0].float()
-    ref = kaldi.fbank(pcm.unsqueeze(0), num_mel_bins=80, frame_length=25, frame_shift=10, dither=0.0,
-                      energy_floor=0.0, sample_frequency=16000)
-    assert (O.fbank(pcm) - ref).abs().max() <= TOL_FBANK
+    shape, frames, ref = _sampled_frames(golden("kaldi_live"), "fbank80_seed77")
+    out = O.fbank(pcm)
+    assert tuple(out.shape) == shape
+    assert (out[frames] - ref).abs().max() <= TOL_FBANK
 
 
 def test_oracle_det_stats_pinned_to_reference_compute_det():
