@@ -167,7 +167,7 @@ WEKWS_API int wekws_model_set_precision(wekws_model* m, int mode);
 WEKWS_API int wekws_model_uses_tensor_cores(const wekws_model* m, int64_t T);
 WEKWS_API int wekws_model_uses_tensor_cores_bt(const wekws_model* m, int64_t B, int64_t T);
 /* Debug/test accessors of the packed host-side program (valid after finalize).      */
-WEKWS_API int64_t wekws_model_packed_floats(const wekws_model* m, int which /*0 stream, 1 vectors, 2 tensor-core weight images (bytes / 4)*/);
+WEKWS_API int64_t wekws_model_packed_floats(const wekws_model* m, int which /*0 stream, 1 vectors, 2 tensor-core weight images (bytes / 4), 3 tensor-core classifier images (bytes / 4)*/);
 WEKWS_API int wekws_model_packed_copy(const wekws_model* m, int which, float* h_dst, int64_t capacity);
 
 /* d_feats (B,T,idim); d_in_cache NULL (start of stream == zeros) or

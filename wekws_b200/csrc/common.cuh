@@ -5,6 +5,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <atomic>
+#include <initializer_list>
 #include <string>
 
 #include "../../include/wekws_b200.h"
@@ -44,6 +45,19 @@ inline int check_launch(const char* what) {
 }
 
 int device_sm_count();
+
+// Raises the dynamic shared-memory limit of `kernels` to `bytes` once per device.  `done` is the launcher's own
+// static per-device flag array: the attribute stays set for the life of the process.
+template <typename... Kernels>
+int set_max_dynamic_smem_once(bool (&done)[64], int bytes, Kernels... kernels) {
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev < 0 || dev >= 64 || done[dev]) return WEKWS_OK;
+  for (const void* k : {(const void*)kernels...})
+    WEKWS_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  done[dev] = true;
+  return WEKWS_OK;
+}
 
 // ---- device helpers ----
 #ifdef __CUDACC__

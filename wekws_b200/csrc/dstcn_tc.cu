@@ -499,13 +499,7 @@ int dstcn_tc_launch(DsTcArgs a, cudaStream_t st) {
   const int tiles = (a.B + a.spt - 1) / a.spt;
   const int grid = tiles < sms ? tiles : sms;
   static bool attr_set[64] = {false};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-    WEKWS_CUDA_OK(cudaFuncSetAttribute(dstcn_tc_kernel<105>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL));
-    WEKWS_CUDA_OK(cudaFuncSetAttribute(dstcn_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL));
-    attr_set[dev] = true;
-  }
+  if (int rc = set_max_dynamic_smem_once(attr_set, SMEM_TOTAL, dstcn_tc_kernel<105>, dstcn_tc_kernel<0>)) return rc;
   if (a.P == 105) dstcn_tc_kernel<105><<<grid, NT_TC, SMEM_TOTAL, st>>>(a);     // ds_tcn.yaml: k = 8, dilations 1, 2, 4, 8
   else dstcn_tc_kernel<0><<<grid, NT_TC, SMEM_TOTAL, st>>>(a);
   return check_launch("dstcn_tc_kernel");

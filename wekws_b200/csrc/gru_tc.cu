@@ -26,6 +26,7 @@
 #include "common.cuh"
 #include "gru_tc.h"
 #include "tc_common.cuh"
+#include "tc_pack.h"
 
 namespace wekws {
 namespace {
@@ -524,20 +525,10 @@ bool gru_tc_eligible(int L, int H_, int idim) { return H_ == H && (L == 1 || L =
 // bf16 image of 128 rows (hidden units) x 64 K (tc_common.cuh layout: row n at n*128, 16-byte chunk c of the slab at
 // chunk c ^ (n & 7)); per K slab a hi chunk then a lo chunk.  Order: Linear; per layer W_hh (r, z, n) then W_ih (r, z, n).
 void gru_tc_pack(uint8_t* dst, const float* wp /*[H][idim]*/, int idim, const float* const* wih /*[L] of [3H][H]*/,
-                 const float* const* whh, int L, uint16_t (*bf16_rn)(float), float (*bf16_to_f)(uint16_t)) {
-  memset(dst, 0, gru_tc_image_bytes(L, idim));
+                 const float* const* whh, int L) {
   uint8_t* p = dst;
   auto slab = [&](const float* W, int ld, int row0, int k0, int kn) {    // rows row0..row0+127, K k0..k0+kn-1
-    uint8_t* hi_img = p;
-    uint8_t* lo_img = p + CHUNK;
-    for (int n = 0; n < H; ++n)
-      for (int kk = 0; kk < kn; ++kk) {
-        const float w = W[(size_t)(row0 + n) * ld + k0 + kk];
-        const uint16_t hi = bf16_rn(w), lo = bf16_rn(w - bf16_to_f(hi));
-        const size_t off = (size_t)n * 128 + (size_t)(((kk >> 3) ^ (n & 7)) << 4) + (size_t)(kk & 7) * 2;
-        memcpy(hi_img + off, &hi, 2);
-        memcpy(lo_img + off, &lo, 2);
-      }
+    write_sw128_image(p, CHUNK, W + (size_t)row0 * ld + k0, H, (size_t)ld, 1, kn);
     p += 2 * CHUNK;
   };
   for (int s = 0; s * 64 < idim; ++s) slab(wp, idim, 0, 64 * s, idim - 64 * s < 64 ? idim - 64 * s : 64);
@@ -558,12 +549,7 @@ int gru_tc_launch(GruTcArgs a, cudaStream_t st) {
   if (const char* e = getenv("WEKWS_GRU_MS")) { const int v = atoi(e); if (v == 16 || v == 32 || v == 64) a.ms = v; }
   a.n_tiles = (a.B + a.ms - 1) / a.ms;
   static bool attr_set[64] = {false};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-    WEKWS_CUDA_OK(cudaFuncSetAttribute(gru_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    attr_set[dev] = true;
-  }
+  if (int rc = set_max_dynamic_smem_once(attr_set, SMEM_BYTES, gru_tc_kernel)) return rc;
   const int sms = device_sm_count();
   const int grid = a.n_tiles < sms ? a.n_tiles : sms;
   gru_tc_kernel<<<grid, NT, SMEM_BYTES, st>>>(a);

@@ -21,8 +21,7 @@ struct GruTcArgs {
 
 size_t gru_tc_image_bytes(int L, int idim);
 bool gru_tc_eligible(int L, int H, int idim);
-void gru_tc_pack(uint8_t* dst, const float* wp, int idim, const float* const* wih, const float* const* whh, int L,
-                 uint16_t (*bf16_rn)(float), float (*bf16_to_f)(uint16_t));
+void gru_tc_pack(uint8_t* dst, const float* wp, int idim, const float* const* wih, const float* const* whh, int L);
 int gru_tc_launch(GruTcArgs a, cudaStream_t st);
 
 }  // namespace wekws

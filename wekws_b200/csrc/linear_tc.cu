@@ -18,6 +18,7 @@
 #include "common.cuh"
 #include "linear_tc.h"
 #include "tc_common.cuh"
+#include "tc_pack.h"
 
 namespace wekws {
 namespace {
@@ -188,20 +189,14 @@ __global__ void __launch_bounds__(NT, 1) linear_tc_kernel(const LinearTcArgs a) 
 size_t linear_tc_image_bytes(int N, int K) { return (size_t)((N + NTILE - 1) / NTILE) * (size_t)(K / 64) * W_SLOT; }
 bool linear_tc_eligible(int N, int K) { return K >= 64 && K <= 256 && K % 64 == 0 && N >= 1; }
 
-void linear_tc_pack(uint8_t* dst, const float* wt, int ldn, int N, int K, uint16_t (*bf16_rn)(float), float (*bf16_to_f)(uint16_t)) {
+void linear_tc_pack(uint8_t* dst, const float* wt, int ldn, int N, int K) {
   const int ntn = (N + NTILE - 1) / NTILE, nslab = K / 64;
-  memset(dst, 0, (size_t)ntn * nslab * W_SLOT);
+  memset(dst, 0, (size_t)ntn * nslab * W_SLOT);          // rows beyond N stay zero
   for (int nt = 0; nt < ntn; ++nt)
     for (int s = 0; s < nslab; ++s) {
-      uint8_t* img = dst + (size_t)(nt * nslab + s) * W_SLOT;      // hi at +0, lo at +16384
-      for (int n = 0; n < NTILE && nt * NTILE + n < N; ++n)
-        for (int kk = 0; kk < 64; ++kk) {
-          const float w = wt[(size_t)(64 * s + kk) * ldn + nt * NTILE + n];
-          const uint16_t hi = bf16_rn(w), lo = bf16_rn(w - bf16_to_f(hi));
-          const size_t off = (size_t)n * 128 + (size_t)(((kk >> 3) ^ (n & 7)) << 4) + (size_t)(kk & 7) * 2;
-          memcpy(img + off, &hi, 2);
-          memcpy(img + 16384 + off, &lo, 2);
-        }
+      const int rows = N - nt * NTILE < NTILE ? N - nt * NTILE : NTILE;
+      write_sw128_image(dst + (size_t)(nt * nslab + s) * W_SLOT, 16384, wt + (size_t)(64 * s) * ldn + nt * NTILE, rows,
+                        1, (size_t)ldn, 64);
     }
 }
 
@@ -211,12 +206,7 @@ int linear_tc_launch(LinearTcArgs a, cudaStream_t st) {
   WEKWS_REQUIRE(((uintptr_t)a.x & 15) == 0 && (a.x_stride & 3) == 0, "linear_tc_launch: input rows must be 16-byte aligned");
   a.n_mtiles = (int)((a.rows + 127) / 128);
   static bool attr_set[64] = {false};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-    WEKWS_CUDA_OK(cudaFuncSetAttribute(linear_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    attr_set[dev] = true;
-  }
+  if (int rc = set_max_dynamic_smem_once(attr_set, SMEM_BYTES, linear_tc_kernel)) return rc;
   const int sms = device_sm_count();
   const int grid = a.n_mtiles < sms ? a.n_mtiles : sms;
   linear_tc_kernel<<<grid, NT, SMEM_BYTES, st>>>(a);

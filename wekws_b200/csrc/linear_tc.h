@@ -19,7 +19,7 @@ struct LinearTcArgs {
 size_t linear_tc_image_bytes(int N, int K);
 bool linear_tc_eligible(int N, int K);
 // wt: W^T as [K][ldn] floats (ldn >= N); writes linear_tc_image_bytes(N, K) bytes
-void linear_tc_pack(uint8_t* dst, const float* wt, int ldn, int N, int K, uint16_t (*bf16_rn)(float), float (*bf16_to_f)(uint16_t));
+void linear_tc_pack(uint8_t* dst, const float* wt, int ldn, int N, int K);
 int linear_tc_launch(LinearTcArgs a, cudaStream_t st);
 
 }  // namespace wekws

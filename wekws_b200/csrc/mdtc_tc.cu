@@ -759,13 +759,7 @@ int mdtc_tc_launch(TcArgs a, int padmax, cudaStream_t st) {
   const int sms = device_sm_count();
   const int grid = a.B < sms ? a.B : sms;
   static bool attr_set[64] = {false};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-    WEKWS_CUDA_OK(cudaFuncSetAttribute(mdtc_tc_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL));
-    WEKWS_CUDA_OK(cudaFuncSetAttribute(mdtc_tc_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL));
-    attr_set[dev] = true;
-  }
+  if (int rc = set_max_dynamic_smem_once(attr_set, SMEM_TOTAL, mdtc_tc_kernel<5>, mdtc_tc_kernel<0>)) return rc;
   if (a.ktaps == 5) mdtc_tc_kernel<5><<<grid, NT_TC, SMEM_TOTAL, st>>>(a);
   else mdtc_tc_kernel<0><<<grid, NT_TC, SMEM_TOTAL, st>>>(a);
   return check_launch("mdtc_tc_kernel");

@@ -23,6 +23,7 @@
 #include "dstcn_tc.h"
 #include "fsmn.h"
 #include "linear_tc.h"
+#include "tc_pack.h"
 
 namespace wekws {
 
@@ -70,6 +71,10 @@ struct Folded {           // BN as per-channel scale/shift
   std::vector<double> s, t;
 };
 
+// A tensor-core kernel: the one pack prepared for a model, or the one a forward call takes (none: the backbone's FP32
+// kernel).
+enum class TcKernel { none, mdtc, tcn, ds_tcn, gru };
+
 }  // namespace
 }  // namespace wekws
 
@@ -80,9 +85,8 @@ struct wekws_model {
   std::map<std::string, std::vector<float>> tensors;
   bool finalized = false;
   int device = 0;
-  int padding = 0, padmax = 0, nblocks = 0;
+  int padmax = 0;                           // widest per-block cache slice of a conv backbone
   bool has_cmvn = false;
-  std::vector<int> dil, coff;
   std::vector<float> h_stream, h_vec;
   std::vector<int> h_chunk_off;
   float* d_stream = nullptr;
@@ -91,17 +95,15 @@ struct wekws_model {
   ConvArgs conv{};
   GruArgs gru{};
   int conv_max_T = 0;
-  // tensor-core path (mdtc, hidden 64)
-  std::vector<std::vector<float>> folded;   // folded GEMM weights W^T [K][64] in consumption order
+  std::vector<std::vector<float>> folded;   // folded GEMM weights W^T [K][C] in consumption order
+  TcKernel tc = TcKernel::none;             // the tensor-core kernel pack prepared: its weight images live in h_wimg / d_wimg
   std::vector<uint8_t> h_wimg;
   uint8_t* d_wimg = nullptr;
-  bool tc_ok = false;
-  int precision = 0;                        // 0 auto (tensor cores where eligible), 1 fp32 FFMA only
-  TcArgs tcargs{};
-  bool tcn_ok = false;                      // tensor-core path for the dense TCN (hidden 64)
-  TcnTcArgs tcnargs{};
-  bool ds_ok = false;                       // tensor-core path for the depthwise-separable TCN (hidden 256)
-  DsTcArgs dsargs{};
+  int precision = 0;                        // 0 auto (tensor cores where eligible), 1 fp32 FFMA only, 2 tensor cores
+  TcArgs tcargs{};                          // mdtc, hidden 64 (mdtc_tc.cu)
+  TcnTcArgs tcnargs{};                      // dense TCN, hidden 64 (tcn_tc.cu)
+  DsTcArgs dsargs{};                        // depthwise-separable TCN, hidden 256 (dstcn_tc.cu)
+  GruTcArgs grutc{};                        // GRU (gru_tc.cu)
   FsmnArgs fsmn{};                          // FSMN backbone (fsmn.cu): weights live in h_vec / d_vec
   bool cls_tc = false;                      // wide classifier head (odim > 4) as its own tcgen05 GEMM (linear_tc.cu)
   std::vector<uint8_t> h_cimg;              //   behind the tensor-core DS-TCN backbone
@@ -110,8 +112,6 @@ struct wekws_model {
   float* d_cbias = nullptr;
   float* d_hidden = nullptr;                // (B, T, 256) scratch between the two kernels; grows monotonically
   size_t hidden_cap = 0;
-  bool gru_tc_ok = false;                   // tensor-core GRU (gru_tc.cu): weight stream lives in h_wimg / d_wimg
-  GruTcArgs grutc{};
 };
 
 namespace {
@@ -198,78 +198,48 @@ int pack_classifier(wekws_model* m, int H, int* v_wc, int* v_bc) {
   return WEKWS_OK;
 }
 
-
-// round-to-nearest-even fp32 -> bf16 (as __floats2bfloat162_rn does on the device)
-uint16_t bf16_rn(float x) {
-  uint32_t u;
-  memcpy(&u, &x, 4);
-  if ((u & 0x7F800000u) == 0x7F800000u) return (uint16_t)(u >> 16);      // inf / nan
-  u += 0x7FFFu + ((u >> 16) & 1u);
-  return (uint16_t)(u >> 16);
-}
-float bf16_to_f(uint16_t h) {
-  uint32_t u = (uint32_t)h << 16;
-  float f;
-  memcpy(&f, &u, 4);
-  return f;
-}
-
-// K-major SWIZZLE_128B image of W[n][k0 .. k0+64) (n < 64): hi at dst, lo at dst + 8192 (tc_common.cuh)
-void write_w_image(uint8_t* dst, const std::vector<float>& wt /*[K][64]*/, int K, int k0) {
-  memset(dst, 0, 16384);
-  for (int n = 0; n < 64; ++n)
-    for (int kk = 0; kk < 64 && k0 + kk < K; ++kk) {
-      const float w = wt[(size_t)(k0 + kk) * 64 + n];
-      const uint16_t hi = bf16_rn(w);
-      const uint16_t lo = bf16_rn(w - bf16_to_f(hi));
-      const size_t off = (size_t)n * 128 + (size_t)(((kk >> 3) ^ (n & 7)) << 4) + (size_t)(kk & 7) * 2;
-      memcpy(dst + off, &hi, 2);
-      memcpy(dst + 8192 + off, &lo, 2);
-    }
+// K-major SWIZZLE_128B image of W[n][k0 .. k0+64) (n < 64) from W^T [K][64]: hi at dst, lo at dst + 8192
+void write_w_image(uint8_t* dst, const std::vector<float>& wt, int K, int k0) {
+  write_sw128_image(dst, 8192, wt.data() + (size_t)k0 * 64, 64, 1, 64, K - k0 < 64 ? K - k0 : 64);
 }
 
 // Same layout for 128 output channels n0 .. n0+127 of a [K][ldn] matrix: hi at dst, lo at dst + 16384 (dstcn_tc.cu)
 void write_w_image128(uint8_t* dst, const std::vector<float>& wt, int ldn, int K, int k0, int n0) {
-  memset(dst, 0, 32768);
-  for (int n = 0; n < 128; ++n)
-    for (int kk = 0; kk < 64 && k0 + kk < K; ++kk) {
-      const float w = wt[(size_t)(k0 + kk) * ldn + n0 + n];
-      const uint16_t hi = bf16_rn(w);
-      const uint16_t lo = bf16_rn(w - bf16_to_f(hi));
-      const size_t off = (size_t)n * 128 + (size_t)(((kk >> 3) ^ (n & 7)) << 4) + (size_t)(kk & 7) * 2;
-      memcpy(dst + off, &hi, 2);
-      memcpy(dst + 16384 + off, &lo, 2);
-    }
+  write_sw128_image(dst, 16384, wt.data() + (size_t)k0 * ldn + n0, 128, 1, (size_t)ldn, K - k0 < 64 ? K - k0 : 64);
+}
+
+// The model fields every tensor-core argument block repeats from ConvArgs, copied by name (the blocks' layouts differ)
+template <typename Args>
+void copy_model_fields(Args& t, const ConvArgs& a) {
+  memset(&t, 0, sizeof(t));
+  t.idim = a.idim; t.odim = a.odim; t.nblocks = a.nblocks; t.ktaps = a.ktaps; t.P = a.P;
+  t.act = a.act; t.has_cmvn = a.has_cmvn;
+  t.v_mean = a.v_mean; t.v_istd = a.v_istd; t.v_bp = a.v_bp; t.v_blocks = a.v_blocks;
+  t.v_blk_stride = a.v_blk_stride; t.v_wc = a.v_wc; t.v_bc = a.v_bc;
+  for (int b = 0; b < a.nblocks; ++b) { t.dil[b] = a.dil[b]; t.coff[b] = a.coff[b]; }
 }
 
 // Tensor-core eligibility + pre-swizzled bf16x3 weight images (mdtc_tc.cu, tcn_tc.cu, dstcn_tc.cu)
 void pack_tc(wekws_model* m) {
-  m->tc_ok = false;
-  m->tcn_ok = false;
-  m->ds_ok = false;
+  m->tc = TcKernel::none;
   m->cls_tc = false;
   m->h_wimg.clear();
   m->h_cimg.clear();
   const wekws_model_config& c = m->cfg;
+  const ConvArgs& a = m->conv;
   if (c.backbone == WEKWS_BACKBONE_DSTCN) {
     DsTcArgs& t = m->dsargs;
-    memset(&t, 0, sizeof(t));
-    const ConvArgs& a = m->conv;
-    t.idim = a.idim; t.odim = a.odim; t.nblocks = a.nblocks; t.ktaps = a.ktaps; t.P = a.P;
-    t.act = a.act; t.has_cmvn = a.has_cmvn;
-    t.v_mean = a.v_mean; t.v_istd = a.v_istd; t.v_bp = a.v_bp; t.v_blocks = a.v_blocks;
-    t.v_blk_stride = a.v_blk_stride; t.v_wc = a.v_wc; t.v_bc = a.v_bc;
-    for (int b = 0; b < a.nblocks; ++b) { t.dil[b] = a.dil[b]; t.coff[b] = a.coff[b]; }
+    copy_model_fields(t, a);
     // output_dim > 4 (CTC vocabularies): the classifier becomes its own tensor-core GEMM fed from a hidden scratch
-    m->cls_tc = c.odim > 4 && linear_tc_eligible(c.odim, c.hdim);
-    t.hidden = m->cls_tc ? reinterpret_cast<float*>(1) : nullptr;      // placeholder for the eligibility test only
+    const bool cls_tc = c.odim > 4 && linear_tc_eligible(c.odim, c.hdim);
+    t.hidden = cls_tc ? reinterpret_cast<float*>(1) : nullptr;      // placeholder for the eligibility test only
     const bool ok = dstcn_tc_eligible(t, c.hdim);
     t.hidden = nullptr;
-    if (!ok) { m->cls_tc = false; return; }
-    if (m->folded.size() != (size_t)(1 + a.nblocks)) { m->cls_tc = false; return; }
-    if (m->cls_tc) {        // W_c^T [256][odim] sits in h_vec at v_wc (pack_classifier), the bias at v_bc
+    if (!ok || m->folded.size() != (size_t)(1 + a.nblocks)) return;
+    m->cls_tc = cls_tc;
+    if (cls_tc) {        // W_c^T [256][odim] sits in h_vec at v_wc (pack_classifier), the bias at v_bc
       m->h_cimg.assign(linear_tc_image_bytes(c.odim, c.hdim), 0);
-      linear_tc_pack(m->h_cimg.data(), m->h_vec.data() + a.v_wc, c.odim, c.odim, c.hdim, bf16_rn, bf16_to_f);
+      linear_tc_pack(m->h_cimg.data(), m->h_vec.data() + a.v_wc, c.odim, c.odim, c.hdim);
       m->h_cbias.assign((size_t)((c.odim + 127) / 128) * 128, 0.f);
       for (int j = 0; j < c.odim; ++j) m->h_cbias[j] = m->h_vec[a.v_bc + j];
     }
@@ -281,45 +251,33 @@ void pack_tc(wekws_model* m) {
     for (int b = 0; b < a.nblocks; ++b)
       for (int ks = 0; ks < 4; ++ks)
         for (int h = 0; h < 2; ++h, dst += 32768) write_w_image128(dst, m->folded[1 + b], 256, 256, 64 * ks, 128 * h);
-    m->ds_ok = true;
+    m->tc = TcKernel::ds_tcn;
     return;
   }
-  if (c.backbone == WEKWS_BACKBONE_TCN && c.hdim == 64) {
+  if (c.hdim != 64) return;
+  if (c.backbone == WEKWS_BACKBONE_TCN) {
     TcnTcArgs& t = m->tcnargs;
-    memset(&t, 0, sizeof(t));
-    const ConvArgs& a = m->conv;
-    t.idim = a.idim; t.odim = a.odim; t.nblocks = a.nblocks; t.ktaps = a.ktaps; t.P = a.P;
-    t.act = a.act; t.has_cmvn = a.has_cmvn;
-    t.v_mean = a.v_mean; t.v_istd = a.v_istd; t.v_bp = a.v_bp; t.v_blocks = a.v_blocks;
-    t.v_blk_stride = a.v_blk_stride; t.v_wc = a.v_wc; t.v_bc = a.v_bc;
-    for (int b = 0; b < a.nblocks; ++b) { t.dil[b] = a.dil[b]; t.coff[b] = a.coff[b]; }
-    if (!tcn_tc_eligible(t, m->padmax)) return;
-    if (m->folded.size() != (size_t)(1 + a.ktaps * a.nblocks)) return;
-    m->h_wimg.assign((size_t)(2 + a.ktaps * a.nblocks) * 16384, 0);
-    write_w_image(m->h_wimg.data(), m->folded[0], a.idim, 0);
-    if (a.idim > 64) write_w_image(m->h_wimg.data() + 16384, m->folded[0], a.idim, 64);
-    for (int g = 0; g < a.ktaps * a.nblocks; ++g)
-      write_w_image(m->h_wimg.data() + (size_t)(2 + g) * 16384, m->folded[1 + g], 64, 0);
-    m->tcn_ok = true;
+    copy_model_fields(t, a);
+    if (!tcn_tc_eligible(t, m->padmax) || m->folded.size() != (size_t)(1 + a.ktaps * a.nblocks)) return;
+    m->tc = TcKernel::tcn;
+  } else if (c.backbone == WEKWS_BACKBONE_MDTC) {
+    TcArgs& t = m->tcargs;
+    copy_model_fields(t, a);
+    t.stack_size = a.stack_size;
+    if (!tc_eligible(t, m->padmax) || m->folded.size() != (size_t)(1 + 2 * a.nblocks)) return;
+    m->tc = TcKernel::mdtc;
+  } else {
     return;
   }
-  if (c.backbone != WEKWS_BACKBONE_MDTC || c.hdim != 64) return;
-  TcArgs& t = m->tcargs;
-  memset(&t, 0, sizeof(t));
-  const ConvArgs& a = m->conv;
-  t.idim = a.idim; t.odim = a.odim; t.nblocks = a.nblocks; t.ktaps = a.ktaps; t.P = a.P;
-  t.stack_size = a.stack_size; t.act = a.act; t.has_cmvn = a.has_cmvn;
-  t.v_mean = a.v_mean; t.v_istd = a.v_istd; t.v_bp = a.v_bp; t.v_blocks = a.v_blocks;
-  t.v_blk_stride = a.v_blk_stride; t.v_wc = a.v_wc; t.v_bc = a.v_bc;
-  for (int b = 0; b < a.nblocks; ++b) { t.dil[b] = a.dil[b]; t.coff[b] = a.coff[b]; }
-  if (!tc_eligible(t, m->padmax)) return;
-  if (m->folded.size() != (size_t)(1 + 2 * a.nblocks)) return;
-  m->h_wimg.assign((size_t)(2 + 2 * a.nblocks) * 16384, 0);
+  // mdtc / tcn: 16 KB images [Wp k 0..63][Wp k 64..127][every further folded GEMM in consumption order]
+  const size_t ngemm = m->folded.size() - 1;
+  m->h_wimg.assign((2 + ngemm) * 16384, 0);
   write_w_image(m->h_wimg.data(), m->folded[0], a.idim, 0);
   if (a.idim > 64) write_w_image(m->h_wimg.data() + 16384, m->folded[0], a.idim, 64);
-  for (int g = 0; g < 2 * a.nblocks; ++g)
-    write_w_image(m->h_wimg.data() + (size_t)(2 + g) * 16384, m->folded[1 + g], 64, 0);
+  for (size_t g = 0; g < ngemm; ++g) write_w_image(m->h_wimg.data() + (2 + g) * 16384, m->folded[1 + g], 64, 0);
+  if (m->tc != TcKernel::mdtc) return;
   // depthwise taps + the two GEMM biases of every block, passed by value with the launch (mdtc_tc.h TcArgs::cw)
+  TcArgs& t = m->tcargs;
   for (int b = 0; b < a.nblocks; ++b) {
     const float* vb = m->h_vec.data() + a.v_blocks + (size_t)b * a.v_blk_stride;
     float* dst = reinterpret_cast<float*>(&t.cw[b][0]);
@@ -336,7 +294,37 @@ void pack_tc(wekws_model* m) {
       dst[6 * 64 + ch] = vb[(a.ktaps + 2) * 64 + ch];
     }
   }
-  m->tc_ok = true;
+}
+
+// Block schedule of the conv backbones: mdtc = preprocessor (dilation 1), then num_stack x stack_size res blocks with
+// dilations 2^l; tcn / ds_tcn = num_layers blocks with dilations 2^i.  Block b (state_dict prefix[b]) keeps
+// dil[b] * (kernel_size - 1) cache columns starting at coff[b]; padding is their total (backbone.padding), padmax the
+// widest slice.
+struct ConvLayout {
+  std::vector<std::string> prefix;
+  std::vector<int> dil, coff;
+  int padding = 0, padmax = 0;
+};
+
+ConvLayout conv_layout(const wekws_model_config& c) {
+  ConvLayout L;
+  auto block = [&](std::string prefix, int dil) {
+    const int pad = dil * (c.kernel_size - 1);
+    L.prefix.push_back(std::move(prefix));
+    L.dil.push_back(dil);
+    L.coff.push_back(L.padding);
+    L.padding += pad;
+    if (pad > L.padmax) L.padmax = pad;
+  };
+  if (c.backbone == WEKWS_BACKBONE_MDTC) {
+    block("backbone.preprocessor", 1);
+    for (int s = 0; s < c.num_stack; ++s)
+      for (int l = 0; l < c.stack_size; ++l)
+        block("backbone.blocks." + std::to_string(s) + ".res_blocks." + std::to_string(l), 1 << l);
+  } else {
+    for (int i = 0; i < c.num_layers; ++i) block("backbone.network." + std::to_string(i) + ".cnn", 1 << i);
+  }
+  return L;
 }
 
 int pack_conv(wekws_model* m) {
@@ -345,33 +333,14 @@ int pack_conv(wekws_model* m) {
   WEKWS_REQUIRE(C == 32 || C == 64 || C == 128 || C == 256, "hidden_dim %d unsupported (32/64/128/256)", C);
   WEKWS_REQUIRE(K >= 2 && K <= 8, "kernel_size %d unsupported (2..8)", K);
   WEKWS_REQUIRE(idim >= 1 && idim <= 128, "input_dim %d unsupported (1..128)", idim);
-  std::vector<std::string> prefix;
-  m->dil.clear(); m->coff.clear();
-  if (c.backbone == WEKWS_BACKBONE_MDTC) {
+  if (c.backbone == WEKWS_BACKBONE_MDTC)
     WEKWS_REQUIRE(c.num_stack >= 1 && c.stack_size >= 1, "mdtc: num_stack/stack_size must be >= 1");
-    prefix.push_back("backbone.preprocessor");
-    m->dil.push_back(1);
-    for (int s = 0; s < c.num_stack; ++s)
-      for (int l = 0; l < c.stack_size; ++l) {
-        prefix.push_back("backbone.blocks." + std::to_string(s) + ".res_blocks." + std::to_string(l));
-        m->dil.push_back(1 << l);
-      }
-  } else {
+  else
     WEKWS_REQUIRE(c.num_layers >= 1, "tcn: num_layers must be >= 1");
-    for (int i = 0; i < c.num_layers; ++i) {
-      prefix.push_back("backbone.network." + std::to_string(i) + ".cnn");
-      m->dil.push_back(1 << i);
-    }
-  }
-  m->nblocks = (int)prefix.size();
-  WEKWS_REQUIRE(m->nblocks <= kMaxBlocks, "%d blocks exceed the supported %d", m->nblocks, kMaxBlocks);
-  m->padding = 0; m->padmax = 0;
-  for (int b = 0; b < m->nblocks; ++b) {
-    m->coff.push_back(m->padding);
-    const int pad = m->dil[b] * (K - 1);
-    m->padding += pad;
-    if (pad > m->padmax) m->padmax = pad;
-  }
+  const ConvLayout layout = conv_layout(c);
+  const int nblocks = (int)layout.dil.size();
+  WEKWS_REQUIRE(nblocks <= kMaxBlocks, "%d blocks exceed the supported %d", nblocks, kMaxBlocks);
+  m->padmax = layout.padmax;
   m->h_stream.clear(); m->h_vec.clear(); m->h_chunk_off.clear(); m->folded.clear();
   ConvArgs& a = m->conv;
   memset(&a, 0, sizeof(a));
@@ -388,8 +357,8 @@ int pack_conv(wekws_model* m) {
   a.v_blocks = (int)m->h_vec.size();
   a.v_blk_stride = c.backbone == WEKWS_BACKBONE_MDTC ? (K + 3) * C
                  : c.backbone == WEKWS_BACKBONE_DSTCN ? (K + 2) * C : C;
-  for (int bi = 0; bi < m->nblocks; ++bi) {
-    const std::string& p = prefix[bi];
+  for (int bi = 0; bi < nblocks; ++bi) {
+    const std::string& p = layout.prefix[bi];
     const size_t v0 = m->h_vec.size();
     if (c.backbone == WEKWS_BACKBONE_MDTC || c.backbone == WEKWS_BACKBONE_DSTCN) {
       const bool md = c.backbone == WEKWS_BACKBONE_MDTC;
@@ -432,11 +401,11 @@ int pack_conv(wekws_model* m) {
   }
   if ((rc = pack_classifier(m, C, &a.v_wc, &a.v_bc))) return rc;
   m->h_chunk_off.push_back((int)m->h_stream.size());
-  a.kind = c.backbone; a.C = C; a.idim = idim; a.odim = c.odim; a.nblocks = m->nblocks; a.ktaps = K;
-  a.P = m->padding; a.stack_size = c.stack_size > 0 ? c.stack_size : 1; a.act = c.activation;
+  a.kind = c.backbone; a.C = C; a.idim = idim; a.odim = c.odim; a.nblocks = nblocks; a.ktaps = K;
+  a.P = layout.padding; a.stack_size = c.stack_size > 0 ? c.stack_size : 1; a.act = c.activation;
   a.has_cmvn = m->has_cmvn ? 1 : 0;
   a.n_chunks = (int)m->h_chunk_off.size() - 1;
-  for (int b = 0; b < m->nblocks; ++b) { a.dil[b] = m->dil[b]; a.coff[b] = m->coff[b]; }
+  for (int b = 0; b < nblocks; ++b) { a.dil[b] = layout.dil[b]; a.coff[b] = layout.coff[b]; }
   pack_tc(m);
   return WEKWS_OK;
 }
@@ -448,7 +417,6 @@ int pack_gru(wekws_model* m) {
   WEKWS_REQUIRE(L >= 1 && L <= 4, "GRU num_layers %d unsupported (1..4)", L);
   WEKWS_REQUIRE(idim >= 1 && idim <= 128, "input_dim %d unsupported (1..128)", idim);
   m->h_stream.clear(); m->h_vec.clear(); m->h_chunk_off.clear();
-  m->padding = 0; m->padmax = 0; m->nblocks = L;
   GruArgs& a = m->gru;
   memset(&a, 0, sizeof(a));
   int rc = pack_common_front(m, &a.v_mean, &a.v_istd);
@@ -478,7 +446,7 @@ int pack_gru(wekws_model* m) {
   if ((rc = pack_classifier(m, H, &a.v_wc, &a.v_bc))) return rc;
   a.L = L; a.H = H; a.idim = idim; a.odim = c.odim; a.act = c.activation; a.has_cmvn = m->has_cmvn ? 1 : 0;
   // tensor-core variant: the per-step weight stream as pre-swizzled bf16 hi|lo operand chunks
-  m->gru_tc_ok = false;
+  m->tc = TcKernel::none;
   m->h_wimg.clear();
   if (gru_tc_eligible(L, H, idim)) {
     const float* wih[4];
@@ -489,13 +457,13 @@ int pack_gru(wekws_model* m) {
       if ((rc = get_tensor(m, "backbone.weight_hh" + sfx, (size_t)G * H, &whh[l]))) return rc;
     }
     m->h_wimg.assign(gru_tc_image_bytes(L, idim), 0);
-    gru_tc_pack(m->h_wimg.data(), wp, idim, wih, whh, L, bf16_rn, bf16_to_f);
+    gru_tc_pack(m->h_wimg.data(), wp, idim, wih, whh, L);
     GruTcArgs& t = m->grutc;
     memset(&t, 0, sizeof(t));
     t.L = L; t.idim = idim; t.odim = c.odim; t.act = c.activation; t.has_cmvn = a.has_cmvn;
     t.v_mean = a.v_mean; t.v_istd = a.v_istd; t.v_bp = a.v_bp; t.v_layers = a.v_layers;
     t.v_layer_stride = a.v_layer_stride; t.v_wc = a.v_wc; t.v_bc = a.v_bc;
-    m->gru_tc_ok = true;
+    m->tc = TcKernel::gru;
   }
   return WEKWS_OK;
 }
@@ -512,7 +480,6 @@ int pack_fsmn(wekws_model* m) {
   WEKWS_REQUIRE(lo >= 1 && ro >= 1, "fsmn: left_order %d / right_order %d unsupported (the reference's FSMNBlock itself "
                 "breaks for right_order = 0: fsmn.py:235 slices x_pad[:, :, :-0])", lo, ro);
   m->h_stream.clear(); m->h_vec.clear(); m->h_chunk_off.clear();
-  m->padding = lo - 1 + ro; m->padmax = m->padding; m->nblocks = L;
   FsmnArgs& a = m->fsmn;
   memset(&a, 0, sizeof(a));
   int rc = pack_common_front(m, &a.o_mean, &a.o_istd);
@@ -617,16 +584,7 @@ extern "C" int wekws_model_padding(const wekws_model* m) {
   if (!m) return 0;
   if (m->cfg.backbone == WEKWS_BACKBONE_GRU) return 0;
   if (m->cfg.backbone == WEKWS_BACKBONE_FSMN) return m->cfg.fsmn_left_order - 1 + m->cfg.fsmn_right_order;
-  int pad = 0;
-  const int K = m->cfg.kernel_size;
-  if (m->cfg.backbone == WEKWS_BACKBONE_MDTC) {
-    pad = K - 1;
-    for (int s = 0; s < m->cfg.num_stack; ++s)
-      for (int l = 0; l < m->cfg.stack_size; ++l) pad += (1 << l) * (K - 1);
-  } else {
-    for (int i = 0; i < m->cfg.num_layers; ++i) pad += (1 << i) * (K - 1);
-  }
-  return pad;
+  return conv_layout(m->cfg).padding;
 }
 
 extern "C" int wekws_model_set_tensor(wekws_model* m, const char* name, const float* h_data, int64_t numel) {
@@ -650,21 +608,24 @@ extern "C" int wekws_model_finalize(wekws_model* m) {
   WEKWS_CUDA_OK(cudaGetDevice(&m->device));
   WEKWS_CUDA_OK(cudaMalloc((void**)&m->d_vec, m->h_vec.size() * sizeof(float)));
   WEKWS_CUDA_OK(cudaMemcpy(m->d_vec, m->h_vec.data(), m->h_vec.size() * sizeof(float), cudaMemcpyHostToDevice));
+  if (m->tc != TcKernel::none) {
+    WEKWS_CUDA_OK(cudaMalloc((void**)&m->d_wimg, m->h_wimg.size()));
+    WEKWS_CUDA_OK(cudaMemcpy(m->d_wimg, m->h_wimg.data(), m->h_wimg.size(), cudaMemcpyHostToDevice));
+  }
   if (m->cfg.backbone == WEKWS_BACKBONE_FSMN) {
     m->fsmn.w = m->d_vec;
-  } else if (m->cfg.backbone != WEKWS_BACKBONE_GRU) {
+  } else if (m->cfg.backbone == WEKWS_BACKBONE_GRU) {
+    m->gru.vec = m->d_vec;
+    m->grutc.vec = m->d_vec; m->grutc.wimg = m->d_wimg;
+  } else {
     WEKWS_CUDA_OK(cudaMalloc((void**)&m->d_stream, m->h_stream.size() * sizeof(float)));
     WEKWS_CUDA_OK(cudaMemcpy(m->d_stream, m->h_stream.data(), m->h_stream.size() * sizeof(float), cudaMemcpyHostToDevice));
     WEKWS_CUDA_OK(cudaMalloc((void**)&m->d_chunk_off, m->h_chunk_off.size() * sizeof(int)));
     WEKWS_CUDA_OK(cudaMemcpy(m->d_chunk_off, m->h_chunk_off.data(), m->h_chunk_off.size() * sizeof(int), cudaMemcpyHostToDevice));
     m->conv.wstream = m->d_stream; m->conv.chunk_off = m->d_chunk_off; m->conv.vec = m->d_vec;
-    if (m->tc_ok || m->tcn_ok || m->ds_ok) {
-      WEKWS_CUDA_OK(cudaMalloc((void**)&m->d_wimg, m->h_wimg.size()));
-      WEKWS_CUDA_OK(cudaMemcpy(m->d_wimg, m->h_wimg.data(), m->h_wimg.size(), cudaMemcpyHostToDevice));
-      m->tcargs.wimg = m->d_wimg; m->tcargs.vec = m->d_vec;
-      m->tcnargs.wimg = m->d_wimg; m->tcnargs.vec = m->d_vec;
-      m->dsargs.wimg = m->d_wimg; m->dsargs.vec = m->d_vec;
-    }
+    m->tcargs.wimg = m->d_wimg; m->tcargs.vec = m->d_vec;
+    m->tcnargs.wimg = m->d_wimg; m->tcnargs.vec = m->d_vec;
+    m->dsargs.wimg = m->d_wimg; m->dsargs.vec = m->d_vec;
     if (m->cls_tc) {
       WEKWS_CUDA_OK(cudaMalloc((void**)&m->d_cimg, m->h_cimg.size()));
       WEKWS_CUDA_OK(cudaMemcpy(m->d_cimg, m->h_cimg.data(), m->h_cimg.size(), cudaMemcpyHostToDevice));
@@ -673,13 +634,6 @@ extern "C" int wekws_model_finalize(wekws_model* m) {
     }
     m->conv_max_T = conv_backbone_max_T(m->conv, m->padmax);
     WEKWS_REQUIRE(m->conv_max_T >= 1, "model does not fit the fused kernel's shared memory");
-  } else {
-    m->gru.vec = m->d_vec;
-    if (m->gru_tc_ok) {
-      WEKWS_CUDA_OK(cudaMalloc((void**)&m->d_wimg, m->h_wimg.size()));
-      WEKWS_CUDA_OK(cudaMemcpy(m->d_wimg, m->h_wimg.data(), m->h_wimg.size(), cudaMemcpyHostToDevice));
-      m->grutc.vec = m->d_vec; m->grutc.wimg = m->d_wimg;
-    }
   }
   m->finalized = true;
   return WEKWS_OK;
@@ -695,15 +649,26 @@ extern "C" int wekws_model_set_precision(wekws_model* m, int mode) {
 // tensor-core kernel takes ~9-10 us per step whatever the batch (up to 148 x 64 streams), the FP32 kernel scales with
 // the streams per SM and has the shorter single-step latency at small batches.
 static bool gru_takes_tc(const wekws_model* m, int64_t B, int64_t T) {
-  if (!m->gru_tc_ok || m->precision == 1 || T < 1) return false;
+  if (m->tc != TcKernel::gru || m->precision == 1 || T < 1) return false;
   if (m->precision == 2) return true;
   return B >= (T == 1 ? 640 : T < 8 ? 400 : 256);
 }
 
+// The kernel a forward call takes: the tensor-core kernel pack prepared, or none (the backbone's FP32 kernel).  The
+// conv kernels need precision != 1, >= 8 frames per call and 16-byte aligned features; mdtc's also 16-byte aligned
+// cache rows (null counts as aligned).
+static TcKernel forward_kernel(const wekws_model* m, int64_t B, int64_t T, const float* feats, const float* in_cache,
+                               const float* out_cache) {
+  auto aligned = [](const float* p) { return ((uintptr_t)p & 15) == 0; };
+  if (m->tc == TcKernel::gru) return gru_takes_tc(m, B, T) ? TcKernel::gru : TcKernel::none;
+  if (m->tc == TcKernel::none || m->precision == 1 || T < 8 || !aligned(feats)) return TcKernel::none;
+  if (m->tc == TcKernel::mdtc && !(aligned(in_cache) && aligned(out_cache))) return TcKernel::none;
+  return m->tc;
+}
+
 extern "C" int wekws_model_uses_tensor_cores_bt(const wekws_model* m, int64_t B, int64_t T) {
   if (!m || !m->finalized) return 0;
-  if (m->cfg.backbone == WEKWS_BACKBONE_GRU) return gru_takes_tc(m, B, T) ? 1 : 0;
-  return ((m->tc_ok || m->tcn_ok || m->ds_ok) && m->precision != 1 && T >= 8) ? 1 : 0;
+  return forward_kernel(m, B, T, nullptr, nullptr, nullptr) != TcKernel::none ? 1 : 0;     // as for aligned tensors
 }
 
 extern "C" int wekws_model_uses_tensor_cores(const wekws_model* m, int64_t T) {
@@ -713,14 +678,16 @@ extern "C" int wekws_model_uses_tensor_cores(const wekws_model* m, int64_t T) {
 extern "C" int64_t wekws_model_packed_floats(const wekws_model* m, int which) {
   if (!m) return 0;
   if (which == 2) return (int64_t)(m->h_wimg.size() / sizeof(float));     // tensor-core weight images, raw bytes
+  if (which == 3) return (int64_t)(m->h_cimg.size() / sizeof(float));     // tensor-core classifier images, raw bytes
   return which == 0 ? (int64_t)m->h_stream.size() : (int64_t)m->h_vec.size();
 }
 
 extern "C" int wekws_model_packed_copy(const wekws_model* m, int which, float* h_dst, int64_t capacity) {
   WEKWS_REQUIRE(m && h_dst, "wekws_model_packed_copy: null argument");
-  if (which == 2) {
-    WEKWS_REQUIRE((int64_t)(m->h_wimg.size() / sizeof(float)) <= capacity, "wekws_model_packed_copy: capacity too small");
-    memcpy(h_dst, m->h_wimg.data(), m->h_wimg.size());
+  if (which == 2 || which == 3) {
+    const std::vector<uint8_t>& img = which == 2 ? m->h_wimg : m->h_cimg;
+    WEKWS_REQUIRE((int64_t)(img.size() / sizeof(float)) <= capacity, "wekws_model_packed_copy: capacity too small");
+    memcpy(h_dst, img.data(), img.size());
     return WEKWS_OK;
   }
   const std::vector<float>& v = which == 0 ? m->h_stream : m->h_vec;
@@ -741,47 +708,24 @@ extern "C" int wekws_model_forward(wekws_model* m, const float* d_feats, const f
   WEKWS_CUDA_OK(cudaGetDevice(&dev));
   WEKWS_REQUIRE(dev == m->device, "model was finalized on device %d but current device is %d", m->device, dev);
   cudaStream_t st = (cudaStream_t)stream;
-  if (m->cfg.backbone == WEKWS_BACKBONE_FSMN) {
-    // time-chunk to the tile height; the cache carries the memory-block state between chunks exactly as in streaming use
-    const int maxT = fsmn_tile_rows();
-    const int nchunk = (int)((T + maxT - 1) / maxT);
-    const int Tc = (int)((T + nchunk - 1) / nchunk);
-    for (int64_t t0 = 0; t0 < T; t0 += Tc) {
-      FsmnArgs a = m->fsmn;
-      a.feats = d_feats + t0 * m->cfg.idim;
-      a.out = d_out + t0 * m->cfg.odim;
-      a.in_cache = t0 == 0 ? d_in_cache : d_out_cache;
-      a.out_cache = d_out_cache;
-      a.B = (int)B;
-      a.T = (int)(T - t0 < Tc ? T - t0 : Tc);
-      a.feat_bstride = T * m->cfg.idim;
-      a.out_bstride = T * m->cfg.odim;
-      int rc = fsmn_launch(a, st);
-      if (rc) return rc;
-    }
-  } else if (m->cfg.backbone == WEKWS_BACKBONE_GRU && gru_takes_tc(m, B, T)) {
-    GruTcArgs a = m->grutc;
-    a.feats = d_feats; a.in_cache = d_in_cache; a.out = d_out; a.out_cache = d_out_cache;
-    a.B = (int)B; a.T = (int)T;
-    int rc = gru_tc_launch(a, st);
-    if (rc) return rc;
-  } else if (m->cfg.backbone == WEKWS_BACKBONE_GRU) {
-    GruArgs a = m->gru;
-    a.feats = d_feats; a.in_cache = d_in_cache; a.out = d_out; a.out_cache = d_out_cache;
-    a.B = (int)B; a.T = (int)T;
-    int rc = gru_launch(a, st);
+  const TcKernel k = forward_kernel(m, B, T, d_feats, d_in_cache, d_out_cache);
+  const bool cls_tc = k == TcKernel::ds_tcn && m->cls_tc;
+  const bool fsmn = m->cfg.backbone == WEKWS_BACKBONE_FSMN;
+  if (m->cfg.backbone == WEKWS_BACKBONE_GRU) {
+    auto call = [&](const auto& model_args) {
+      auto a = model_args;
+      a.feats = d_feats; a.in_cache = d_in_cache; a.out = d_out; a.out_cache = d_out_cache;
+      a.B = (int)B; a.T = (int)T;
+      return a;
+    };
+    int rc = k == TcKernel::gru ? gru_tc_launch(call(m->grutc), st) : gru_launch(call(m->gru), st);
     if (rc) return rc;
   } else {
     // time-chunk long inputs; the cache carries the state between chunks exactly as in
     // streaming use (chunked == full utterance, SURVEY.md 8a "Numerical facts")
-    // tensor-core path: mdtc hidden 64, chunks of >= 8 frames, 16-byte aligned cache rows
-    const bool use_tc = m->tc_ok && m->precision != 1 && T >= 8 &&
-                        (d_in_cache == nullptr || ((uintptr_t)d_in_cache & 15) == 0) &&
-                        ((uintptr_t)d_feats & 15) == 0 && ((uintptr_t)d_out_cache & 15) == 0;
-    const bool use_tcn = m->tcn_ok && m->precision != 1 && T >= 8 && ((uintptr_t)d_feats & 15) == 0;
-    const bool use_ds = m->ds_ok && m->precision != 1 && T >= 8 && ((uintptr_t)d_feats & 15) == 0;
-    const int maxT = use_tc ? tc_max_T() : use_tcn ? tcn_tc_max_T() : use_ds ? dstcn_tc_max_T() : m->conv_max_T;
-    if (use_ds && m->cls_tc) {      // hidden scratch between the backbone kernel and the classifier GEMM
+    const int maxT = k == TcKernel::mdtc ? tc_max_T() : k == TcKernel::tcn ? tcn_tc_max_T()
+                   : k == TcKernel::ds_tcn ? dstcn_tc_max_T() : fsmn ? fsmn_tile_rows() : m->conv_max_T;
+    if (cls_tc) {      // hidden scratch between the backbone kernel and the classifier GEMM
       const size_t need = (size_t)B * (size_t)T * (size_t)m->cfg.hdim;
       if (need > m->hidden_cap) {
         WEKWS_CUDA_OK(cudaStreamSynchronize(st));          // the old scratch may still be in use on this stream
@@ -794,8 +738,9 @@ extern "C" int wekws_model_forward(wekws_model* m, const float* d_feats, const f
     const int nchunk = (int)((T + maxT - 1) / maxT);
     const int Tc = (int)((T + nchunk - 1) / nchunk);
     for (int64_t t0 = 0; t0 < T; t0 += Tc) {
-      if (use_tc) {
-        TcArgs a = m->tcargs;
+      // the per-chunk fields of every chunked kernel's argument block, set by name (the blocks' layouts differ)
+      auto chunk = [&](const auto& model_args) {
+        auto a = model_args;
         a.feats = d_feats + t0 * m->cfg.idim;
         a.out = d_out + t0 * m->cfg.odim;
         a.in_cache = t0 == 0 ? d_in_cache : d_out_cache;
@@ -804,54 +749,24 @@ extern "C" int wekws_model_forward(wekws_model* m, const float* d_feats, const f
         a.T = (int)(T - t0 < Tc ? T - t0 : Tc);
         a.feat_bstride = T * m->cfg.idim;
         a.out_bstride = T * m->cfg.odim;
-        int rc = mdtc_tc_launch(a, m->padmax, st);
-        if (rc) return rc;
-        continue;
+        return a;
+      };
+      int rc;
+      switch (k) {
+        case TcKernel::mdtc: rc = mdtc_tc_launch(chunk(m->tcargs), m->padmax, st); break;
+        case TcKernel::tcn: rc = tcn_tc_launch(chunk(m->tcnargs), m->padmax, st); break;
+        case TcKernel::ds_tcn: {
+          DsTcArgs a = chunk(m->dsargs);
+          if (cls_tc) { a.hidden = m->d_hidden + t0 * m->cfg.hdim; a.hidden_bstride = T * m->cfg.hdim; }
+          rc = dstcn_tc_launch(a, st);
+          break;
+        }
+        default: rc = fsmn ? fsmn_launch(chunk(m->fsmn), st) : conv_backbone_launch(chunk(m->conv), m->padmax, st);
       }
-      if (use_ds) {
-        DsTcArgs a = m->dsargs;
-        a.feats = d_feats + t0 * m->cfg.idim;
-        a.out = d_out + t0 * m->cfg.odim;
-        a.in_cache = t0 == 0 ? d_in_cache : d_out_cache;
-        a.out_cache = d_out_cache;
-        a.B = (int)B;
-        a.T = (int)(T - t0 < Tc ? T - t0 : Tc);
-        a.feat_bstride = T * m->cfg.idim;
-        a.out_bstride = T * m->cfg.odim;
-        if (m->cls_tc) { a.hidden = m->d_hidden + t0 * m->cfg.hdim; a.hidden_bstride = T * m->cfg.hdim; }
-        int rc = dstcn_tc_launch(a, st);
-        if (rc) return rc;
-        continue;
-      }
-      if (use_tcn) {
-        TcnTcArgs a = m->tcnargs;
-        a.feats = d_feats + t0 * m->cfg.idim;
-        a.out = d_out + t0 * m->cfg.odim;
-        a.in_cache = t0 == 0 ? d_in_cache : d_out_cache;
-        a.out_cache = d_out_cache;
-        a.B = (int)B;
-        a.T = (int)(T - t0 < Tc ? T - t0 : Tc);
-        a.feat_bstride = T * m->cfg.idim;
-        a.out_bstride = T * m->cfg.odim;
-        int rc = tcn_tc_launch(a, m->padmax, st);
-        if (rc) return rc;
-        continue;
-      }
-      ConvArgs a = m->conv;
-      a.feats = d_feats + t0 * m->cfg.idim;
-      a.out = d_out + t0 * m->cfg.odim;
-      a.in_cache = t0 == 0 ? d_in_cache : d_out_cache;
-      a.out_cache = d_out_cache;
-      a.B = (int)B;
-      a.T = (int)(T - t0 < Tc ? T - t0 : Tc);
-      a.feat_bstride = T * m->cfg.idim;
-      a.out_bstride = T * m->cfg.odim;
-      int rc = conv_backbone_launch(a, m->padmax, st);
       if (rc) return rc;
     }
   }
-  if (m->cfg.backbone == WEKWS_BACKBONE_DSTCN && m->cls_tc && m->ds_ok && m->precision != 1 && T >= 8 &&
-      ((uintptr_t)d_feats & 15) == 0) {
+  if (cls_tc) {
     // classifier (+ activation) of all B*T frames in one tensor-core GEMM over the hidden scratch (classifier.py:63-67)
     LinearTcArgs a;
     a.x = m->d_hidden; a.out = d_out; a.wimg = m->d_cimg; a.bias = m->d_cbias;

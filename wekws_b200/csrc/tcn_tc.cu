@@ -459,12 +459,7 @@ int tcn_tc_launch(TcnTcArgs a, int padmax, cudaStream_t st) {
   const int sms = device_sm_count();
   const int grid = a.B < sms ? a.B : sms;
   static bool attr_set[64] = {false};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-    WEKWS_CUDA_OK(cudaFuncSetAttribute(tcn_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_TOTAL));
-    attr_set[dev] = true;
-  }
+  if (int rc = set_max_dynamic_smem_once(attr_set, SMEM_TOTAL, tcn_tc_kernel)) return rc;
   tcn_tc_kernel<<<grid, NT_TC, SMEM_TOTAL, st>>>(a);
   return check_launch("tcn_tc_kernel");
 }

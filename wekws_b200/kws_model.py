@@ -292,6 +292,35 @@ class KWSModel(nn.Module):
 
 
     # ------------------------------------------------------------------------- forward
+    def _prepare_call(self, dev: torch.device, B: int, T: int, in_cache: torch.Tensor):
+        """What every native forward (``model(feats)`` and ``Pipeline``) needs for B streams of T frames on `dev`: the
+        handle, packed and with the precision applied; the input cache as a contiguous fp32 tensor on `dev` (None: start
+        of stream; the caller keeps it alive until the launch); the output tensors.  For T == 0 the output cache is the
+        input cache (or zeros)."""
+        if isinstance(self.backbone, nn.GRU):
+            cache_shape = (self.backbone.num_layers, B, self.hdim)
+        elif getattr(self.backbone, "kind", None) == "fsmn":      # 4-D: one column block per layer (fsmn.py:488)
+            cache_shape = (B, self.backbone.proj_dim, self.backbone.cache_len, self.backbone.fsmn_layers)
+        else:
+            cache_shape = (B, self.hdim, self.backbone.padding)
+        if in_cache is not None and in_cache.numel() > 0:
+            if tuple(in_cache.shape) != cache_shape:
+                raise ValueError(f"in_cache must be {cache_shape}, got {tuple(in_cache.shape)}")
+            if in_cache.device != dev or in_cache.dtype != torch.float32 or not in_cache.is_contiguous():
+                in_cache = in_cache.to(device=dev, dtype=torch.float32).contiguous()
+        else:
+            in_cache = None
+        h = self._ensure(dev)
+        self._apply_precision(h)
+        out = torch.empty((B, T, self.odim), device=dev, dtype=torch.float32)
+        if T == 0 and in_cache is not None:
+            out_cache = in_cache.clone()
+        elif T == 0:
+            out_cache = torch.zeros(cache_shape, device=dev, dtype=torch.float32)
+        else:
+            out_cache = torch.empty(cache_shape, device=dev, dtype=torch.float32)
+        return h, in_cache, out, out_cache
+
     def _run(self, x: torch.Tensor, in_cache: torch.Tensor, flags: int) -> Tuple[torch.Tensor, torch.Tensor]:
         if self.training:
             raise RuntimeError("wekws_b200.KWSModel is inference-only: call model.eval() first "
@@ -307,29 +336,8 @@ class KWSModel(nn.Module):
         B, T = x.size(0), x.size(1)
         if not x.is_contiguous():
             x = x.contiguous()
-        gru = isinstance(self.backbone, nn.GRU)
-        if gru:
-            cache_shape = (self.backbone.num_layers, B, self.hdim)
-        elif getattr(self.backbone, "kind", None) == "fsmn":      # 4-D: one column block per layer (fsmn.py:488)
-            cache_shape = (B, self.backbone.proj_dim, self.backbone.cache_len, self.backbone.fsmn_layers)
-        else:
-            cache_shape = (B, self.hdim, self.backbone.padding)
-        cache_ptr = None
-        if in_cache is not None and in_cache.numel() > 0:
-            if tuple(in_cache.shape) != cache_shape:
-                raise ValueError(f"in_cache must be {cache_shape}, got {tuple(in_cache.shape)}")
-            if in_cache.device != dev or in_cache.dtype != torch.float32 or not in_cache.is_contiguous():
-                in_cache = in_cache.to(device=dev, dtype=torch.float32).contiguous()
-            cache_ptr = in_cache.data_ptr()
-        h = self._ensure(dev)
-        self._apply_precision(h)
-        out = torch.empty((B, T, self.odim), device=dev, dtype=torch.float32)
-        if T == 0 and cache_ptr is not None:
-            out_cache = in_cache.clone()
-        elif T == 0:
-            out_cache = torch.zeros(cache_shape, device=dev, dtype=torch.float32)
-        else:
-            out_cache = torch.empty(cache_shape, device=dev, dtype=torch.float32)
+        h, in_cache, out, out_cache = self._prepare_call(dev, B, T, in_cache)
+        cache_ptr = None if in_cache is None else in_cache.data_ptr()
         if B > 0 and T > 0:
             fwd = _native.lib().wekws_model_forward
             if torch.cuda.current_device() == dev.index:          # common case: no device switch needed

@@ -12,7 +12,6 @@ import ctypes as C
 from typing import Tuple
 
 import torch
-import torch.nn as nn
 
 from . import _native
 from .frontend import Fbank
@@ -40,32 +39,14 @@ class Pipeline:
         dev = pcm.device
         B, N = pcm.shape
         T = fe.num_frames(N)
-        gru = isinstance(m.backbone, nn.GRU)
-        if gru:
-            cache_shape = (m.backbone.num_layers, B, m.hdim)
-        elif getattr(m.backbone, "kind", None) == "fsmn":
-            cache_shape = (B, m.backbone.proj_dim, m.backbone.cache_len, m.backbone.fsmn_layers)
-        else:
-            cache_shape = (B, m.hdim, m.backbone.padding)
-        cache_ptr = None
-        if in_cache is not None and in_cache.numel() > 0:
-            if tuple(in_cache.shape) != cache_shape:
-                raise ValueError(f"in_cache must be {cache_shape}, got {tuple(in_cache.shape)}")
-            in_cache = in_cache.to(device=dev, dtype=torch.float32).contiguous()
-            cache_ptr = in_cache.data_ptr()
-        out = torch.empty((B, T, m.odim), device=dev, dtype=torch.float32)
+        h_model, in_cache, out, out_cache = m._prepare_call(dev, B, T, in_cache)
+        cache_ptr = None if in_cache is None else in_cache.data_ptr()
         if T == 0 or B == 0:
-            return out, (in_cache.clone() if cache_ptr is not None else torch.zeros(cache_shape, device=dev))
-        out_cache = torch.empty(cache_shape, device=dev, dtype=torch.float32)
+            return out, out_cache
         need = B * T * m.idim
         if self._scratch is None or self._scratch.numel() < need or self._scratch.device != dev:
             self._scratch = torch.empty(need, device=dev, dtype=torch.float32)
         with torch.cuda.device(dev):
-            h_model = m._ensure(dev)
-            if m._precision_applied != m.precision:
-                _native.check(_native.lib().wekws_model_set_precision(h_model, 0 if m.precision == "auto" else 1),
-                              "wekws_model_set_precision")
-                m._precision_applied = m.precision
             rc = _native.lib().wekws_pipeline_forward(
                 fe._handle(dev), h_model, C.c_void_p(pcm.data_ptr()),
                 _native.PCM_S16 if pcm.dtype == torch.int16 else _native.PCM_F32, B, N, pcm.stride(0),
