@@ -29,6 +29,9 @@
  *   wekws_pipeline_forward the composition the callers perform: Fbank -> model, i.e.
  *                          stream_kws_ctc.py:482-487 / score.py:117-127, raw PCM in,
  *                          posteriors out.
+ *   wekws_kws_*            the streaming CTC keyword spotter around them: KeyWordSpotter
+ *                          wekws/bin/stream_kws_ctc.py:218-529 (PCM / feature carries,
+ *                          per-frame beam step + execute_detection, reset / reset_all).
  */
 #ifndef WEKWS_B200_H_
 #define WEKWS_B200_H_
@@ -40,7 +43,7 @@
 extern "C" {
 #endif
 
-#define WEKWS_B200_ABI_VERSION 4   /* 2: + wekws_fbank_set_mfcc, wekws_fbank_feature_dim, wekws_det_stats; 3: det max_score is double; 4: precision mode 2, wekws_model_uses_tensor_cores_bt */
+#define WEKWS_B200_ABI_VERSION 5   /* 2: + wekws_fbank_set_mfcc, wekws_fbank_feature_dim, wekws_det_stats; 3: det max_score is double; 4: precision mode 2, wekws_model_uses_tensor_cores_bt; 5: + wekws_kws_* streaming keyword spotter */
 
 #if defined(__GNUC__)
 #define WEKWS_API __attribute__((visibility("default")))
@@ -227,6 +230,56 @@ WEKWS_API int wekws_ctc_keyword_hit(const int32_t* d_nhyp, const int32_t* d_hyp_
 WEKWS_API int64_t wekws_context_expand_frames(int64_t num_frames, int right, int skip);
 WEKWS_API int wekws_context_expand(const float* d_feats, const int32_t* d_lens, int64_t B, int64_t T, int D, int left,
                          int right, int skip, float* d_out, int64_t out_frames, void* stream);
+
+/* ------------------------------------------------------------------ streaming CTC keyword spotter
+ * KeyWordSpotter of wekws/bin/stream_kws_ctc.py:218-529 for B streams at once, bit-exact (wekws_b200/spotter.py drives
+ * it).  The host plans every row count and offset from the sample counts it knows; nothing here is read back to plan.
+ *
+ * wekws_kws_splice  accept_wave :346-364: stage[b] = carry_in[b][0..carry_len) ++ pcm[b][0..new_len) (int16, row
+ *   stride stage_stride, for wekws_fbank_forward with d_lens = carry_len + new_len), and carry_out[b] = stage[b] from
+ *   sample consumed[b] on (the samples the Fbank frames did not use).  carry_in / carry_out: (B, carry_cap), distinct.
+ * wekws_kws_context accept_wave :366-397: d_feats (B,T,D) Fbank rows, d_num_frames (B) rows per stream.  With expand,
+ *   the rows are context-expanded with the carried rows d_carry_in (B, left+right, D), d_carry_len (B) rows (-1 =
+ *   first chunk: left copies of row 0), and the next carry is written to d_carry_out (the last min(left+right, nf) rows;
+ *   the old carry when nf == 0).  Then every skip-th row from d_skip_offset[b] on is written to d_out at packed row
+ *   d_row_offsets[b], d_rows[b] rows (width D*(left+right+1) with expand, D without); max_rows = max of d_rows.
+ * wekws_kws_detect  forward :489-512: per stream d_rows[b] rows of softmax posteriors at d_probs + d_row_offsets[b]*V,
+ *   each one streaming beam step (wekws_ctc_prefix_beam_search's) then execute_detection :411-480; after an activation
+ *   the beam is reset and the rest of the chunk is skipped; at the end of the chunk a top hypothesis whose first token
+ *   is more than max_frames old is reset.  d_token_set: keywords_idxset; d_kw_tokens / d_kw_offsets as in
+ *   wekws_ctc_keyword_hit, in dict order.  d_state: B x wekws_kws_state_bytes(), set up by wekws_kws_reset(full = 1).
+ *   d_result (B, WEKWS_KWS_RESULT_FIELDS) int64: state (-1 = no rows: the reference returns {}, 0, 1 = activated),
+ *   keyword index (-1), start frame, end frame, score (the bits of the double hit_score), overflow (a prefix outgrew
+ *   WEKWS_CTC_MAX_PREFIX tokens or the node pool filled since the last full reset; the results are then not exact).
+ * wekws_kws_reset   reset() :516-519 (full = 0) or the decoder part of reset_all() :521-529 (full = 1: also
+ *   total_frames, last_active_pos, the overflow flag) of the listed streams (d_streams NULL: streams 0..B-1).       */
+#define WEKWS_KWS_RESULT_FIELDS 6
+typedef struct {
+  double threshold;          /* activation: hit_score >= threshold                                           */
+  int32_t min_frames;        /* and min_frames <= end - start <= max_frames                                  */
+  int32_t max_frames;
+  int32_t interval_frames;   /* and (no activation yet or end - last_active_pos >= interval_frames)          */
+  int32_t score_beam;        /* 1..WEKWS_CTC_MAX_SCORE_BEAM                                                  */
+  int32_t path_beam;         /* 1..WEKWS_CTC_MAX_PATH_BEAM                                                   */
+  int32_t frame_skip;        /* row t of a chunk is frame total_frames + t * frame_skip                      */
+} wekws_kws_config;
+
+WEKWS_API int64_t wekws_kws_state_bytes(void);
+WEKWS_API int wekws_kws_reset(void* d_state, int64_t B, const int32_t* d_streams, int64_t n_streams, int full,
+                              void* stream);
+WEKWS_API int wekws_kws_detect(const float* d_probs, const int32_t* d_row_offsets, const int32_t* d_rows, int64_t B,
+                               int V, const int32_t* d_token_set, int n_tokens, const int32_t* d_kw_tokens,
+                               const int32_t* d_kw_offsets, int num_keywords, const wekws_kws_config* cfg,
+                               void* d_state, int64_t* d_result, void* stream);
+WEKWS_API int wekws_kws_splice(const int16_t* d_pcm, int64_t pcm_stride, const int32_t* d_new_len,
+                               const int32_t* d_carry_len, const int32_t* d_consumed, const int16_t* d_carry_in,
+                               int16_t* d_carry_out, int64_t carry_cap, int16_t* d_stage, int64_t stage_stride,
+                               int64_t B, void* stream);
+WEKWS_API int wekws_kws_context(const float* d_feats, int64_t B, int64_t T, int D, const int32_t* d_num_frames,
+                                const float* d_carry_in, const int32_t* d_carry_len, float* d_carry_out, int left,
+                                int right, int expand, int skip, const int32_t* d_skip_offset,
+                                const int32_t* d_row_offsets, const int32_t* d_rows, int64_t max_rows, float* d_out,
+                                void* stream);
 
 /* Raw PCM -> posteriors: Fbank(+CMVN from the model's global_cmvn.* if set) -> model.
  * d_feat_scratch: (B, frames, idim) floats of workspace owned by the caller.        */

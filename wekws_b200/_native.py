@@ -18,7 +18,8 @@ BACKBONE_MDTC, BACKBONE_TCN, BACKBONE_DSTCN, BACKBONE_GRU, BACKBONE_FSMN = 0, 1,
 ACT_IDENTITY, ACT_SIGMOID = 0, 1
 PCM_S16, PCM_F32 = 0, 1
 FWD_SOFTMAX = 1
-ABI_VERSION = 4
+ABI_VERSION = 5
+KWS_RESULT_FIELDS = 6
 
 
 class FbankConfig(C.Structure):
@@ -34,6 +35,12 @@ class ModelConfig(C.Structure):
                 ("fsmn_input_affine_dim", C.c_int32), ("fsmn_linear_dim", C.c_int32), ("fsmn_proj_dim", C.c_int32),
                 ("fsmn_left_order", C.c_int32), ("fsmn_right_order", C.c_int32),
                 ("fsmn_output_affine_dim", C.c_int32)]
+
+
+class KwsConfig(C.Structure):
+    _fields_ = [("threshold", C.c_double), ("min_frames", C.c_int32), ("max_frames", C.c_int32),
+                ("interval_frames", C.c_int32), ("score_beam", C.c_int32), ("path_beam", C.c_int32),
+                ("frame_skip", C.c_int32)]
 
 
 # name -> (restype, argtypes); every symbol include/wekws_b200.h declares
@@ -75,6 +82,16 @@ SIGNATURES = {
     "wekws_context_expand_frames": (C.c_int64, [C.c_int64, C.c_int, C.c_int]),
     "wekws_context_expand": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int,
                                        C.c_void_p, C.c_int64, C.c_void_p]),
+    "wekws_kws_state_bytes": (C.c_int64, []),
+    "wekws_kws_reset": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
+    "wekws_kws_detect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_int,
+                                   C.c_void_p, C.c_void_p, C.c_int, C.POINTER(KwsConfig), C.c_void_p, C.c_void_p,
+                                   C.c_void_p]),
+    "wekws_kws_splice": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]),
+    "wekws_kws_context": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.c_int64, C.c_void_p, C.c_void_p]),
     "wekws_pipeline_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64,
                                          C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_uint32, C.c_void_p]),
