@@ -32,6 +32,9 @@
  *   wekws_kws_*            the streaming CTC keyword spotter around them: KeyWordSpotter
  *                          wekws/bin/stream_kws_ctc.py:218-529 (PCM / feature carries,
  *                          per-frame beam step + execute_detection, reset / reset_all).
+ *   wekws_ctc_stream_score the test-set scorer wekws/bin/stream_score_ctc.py:209-381 (per
+ *                          utterance: per-frame beam step + the script's own detection).
+ *   wekws_ctc_det_sweep    the threshold sweep of wekws/bin/compute_det_ctc.py:251-281.
  */
 #ifndef WEKWS_B200_H_
 #define WEKWS_B200_H_
@@ -43,7 +46,7 @@
 extern "C" {
 #endif
 
-#define WEKWS_B200_ABI_VERSION 5   /* 2: + wekws_fbank_set_mfcc, wekws_fbank_feature_dim, wekws_det_stats; 3: det max_score is double; 4: precision mode 2, wekws_model_uses_tensor_cores_bt; 5: + wekws_kws_* streaming keyword spotter */
+#define WEKWS_B200_ABI_VERSION 6   /* 2: + wekws_fbank_set_mfcc, wekws_fbank_feature_dim, wekws_det_stats; 3: det max_score is double; 4: precision mode 2, wekws_model_uses_tensor_cores_bt; 5: + wekws_kws_* streaming keyword spotter; 6: + wekws_ctc_stream_score, wekws_ctc_det_sweep */
 
 #if defined(__GNUC__)
 #define WEKWS_API __attribute__((visibility("default")))
@@ -280,6 +283,35 @@ WEKWS_API int wekws_kws_context(const float* d_feats, int64_t B, int64_t T, int 
                                 int right, int expand, int skip, const int32_t* d_skip_offset,
                                 const int32_t* d_row_offsets, const int32_t* d_rows, int64_t max_rows, float* d_out,
                                 void* stream);
+
+/* ------------------------------------------------------------------ CTC test-set scoring and DET statistics
+ * wekws_ctc_stream_score  wekws/bin/stream_score_ctc.py:209-381 for B utterances, bit-exact: d_probs (B,T,V) softmax
+ *   posteriors, d_lens (B) valid rows (NULL = T; values outside [0, T] are clamped), row t is frame t * frame_skip.
+ *   d_token_set: keywords_idxset (n_tokens = 0: no filter); d_kw_tokens / d_kw_offsets as in wekws_ctc_keyword_hit,
+ *   in dict order.  Per utterance: d_count (B) activations (always exact), d_overflow (B) != 0 if a prefix outgrew
+ *   WEKWS_CTC_MAX_PREFIX tokens or the node pool filled (the results are then not exact), and the first
+ *   min(count, max_detections) activations in frame order in d_kw / d_score (double hit_score) / d_start / d_end,
+ *   each (B, max_detections).
+ * wekws_ctc_det_sweep  compute_det_ctc.py:251-281 for one keyword: d_false_reject[i] = #(d_conf_kw < thr[i]),
+ *   d_false_alarm[i] = #(d_conf_filler >= thr[i]), compared in double; d_thresholds as the host accumulates them. */
+typedef struct {
+  double threshold;          /* activation: hit_score >= threshold                                           */
+  int32_t min_frames;        /* and min_frames <= end - start <= max_frames                                  */
+  int32_t max_frames;
+  int32_t score_beam;        /* 1..WEKWS_CTC_MAX_SCORE_BEAM                                                  */
+  int32_t path_beam;         /* 1..WEKWS_CTC_MAX_PATH_BEAM                                                   */
+  int32_t frame_skip;        /* dataset_conf.frame_skip: row t is frame t * frame_skip                       */
+  int32_t max_detections;    /* >= 1: detections stored per utterance                                        */
+} wekws_ctc_score_config;
+
+WEKWS_API int wekws_ctc_stream_score(const float* d_probs, const int32_t* d_lens, int64_t B, int64_t T, int V,
+                                     const int32_t* d_token_set, int n_tokens, const int32_t* d_kw_tokens,
+                                     const int32_t* d_kw_offsets, int num_keywords, const wekws_ctc_score_config* cfg,
+                                     int32_t* d_count, int32_t* d_overflow, int32_t* d_kw, double* d_score,
+                                     int32_t* d_start, int32_t* d_end, void* stream);
+WEKWS_API int wekws_ctc_det_sweep(const double* d_conf_kw, int64_t n_kw, const double* d_conf_filler, int64_t n_filler,
+                                  const double* d_thresholds, int nthr, int64_t* d_false_reject,
+                                  int64_t* d_false_alarm, void* stream);
 
 /* Raw PCM -> posteriors: Fbank(+CMVN from the model's global_cmvn.* if set) -> model.
  * d_feat_scratch: (B, frames, idim) floats of workspace owned by the caller.        */

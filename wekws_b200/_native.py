@@ -18,7 +18,7 @@ BACKBONE_MDTC, BACKBONE_TCN, BACKBONE_DSTCN, BACKBONE_GRU, BACKBONE_FSMN = 0, 1,
 ACT_IDENTITY, ACT_SIGMOID = 0, 1
 PCM_S16, PCM_F32 = 0, 1
 FWD_SOFTMAX = 1
-ABI_VERSION = 5
+ABI_VERSION = 6
 KWS_RESULT_FIELDS = 6
 
 
@@ -41,6 +41,12 @@ class KwsConfig(C.Structure):
     _fields_ = [("threshold", C.c_double), ("min_frames", C.c_int32), ("max_frames", C.c_int32),
                 ("interval_frames", C.c_int32), ("score_beam", C.c_int32), ("path_beam", C.c_int32),
                 ("frame_skip", C.c_int32)]
+
+
+class CtcScoreConfig(C.Structure):
+    _fields_ = [("threshold", C.c_double), ("min_frames", C.c_int32), ("max_frames", C.c_int32),
+                ("score_beam", C.c_int32), ("path_beam", C.c_int32), ("frame_skip", C.c_int32),
+                ("max_detections", C.c_int32)]
 
 
 # name -> (restype, argtypes); every symbol include/wekws_b200.h declares
@@ -92,6 +98,11 @@ SIGNATURES = {
     "wekws_kws_context": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_int64, C.c_void_p, C.c_void_p]),
+    "wekws_ctc_stream_score": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_int,
+                                         C.c_void_p, C.c_void_p, C.c_int, C.POINTER(CtcScoreConfig), C.c_void_p,
+                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "wekws_ctc_det_sweep": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_void_p,
+                                      C.c_void_p, C.c_void_p]),
     "wekws_pipeline_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64,
                                          C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_uint32, C.c_void_p]),
